@@ -3,9 +3,11 @@
     python bench.py --gpus 1 --steps 10 --warmup 3
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
     python bench.py --impl reference ...      # the CPU arm: the oracle port timed on the host cores
+    python bench.py ... --dump-outputs DIR    # also write what the last timed step computed, as DIR/<name>.npy
 
 A "step" is one pass of the hot path over one synthetic batch: forward + loss + backward + (DDP gradient all-reduce) +
 clip/AdamW/apply_every, i.e. one iteration of the reference's inner loop (train.py:186-190).  Prints ONE JSON line.
+Inputs and parameters are seeded, so two builds run with the same arguments can be compared dump for dump.
 """
 import argparse
 import json
@@ -21,6 +23,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the tree as it found it (no __pycache__ for the project's modules)
 
 CONFIGS = {
     # BASELINE.json configs[1]: the configuration the metric is quoted on
@@ -113,6 +116,32 @@ def synthetic_batches(count, B, n, seed):
         t = torch.from_numpy(rng.integers(0, 256, (B, n + 1)).astype(np.int32))
         out.append(t.pin_memory() if torch.cuda.is_available() else t)
     return out
+
+
+DUMP_SAMPLE = 1 << 21    # elements kept of a larger output: three 8 MB float32 samples stay well inside 64 MB per dump
+
+
+def dump_sample(x, seed):
+    """x flattened to float32; above DUMP_SAMPLE elements, a fixed subset whose indices depend only on `seed` and x.size"""
+    x = np.asarray(x, np.float32).ravel()
+    if x.size <= DUMP_SAMPLE:
+        return x
+    return x[np.sort(np.random.default_rng(seed).integers(0, x.size, DUMP_SAMPLE))]
+
+
+def dump_outputs(path, arrays):
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + '.npy'), a)
+
+
+def train_step_outputs(eng, loss):
+    """What the last timed training step computed: its loss, its logits, the parameter gradient and the parameters after
+    the optimizer update.  Trees are flattened in sorted (module, name) order, so the sample does not depend on the
+    engine's internal buffer layout."""
+    flat = lambda tree: np.concatenate([tree[m][k].ravel() for m in sorted(tree) for k in sorted(tree[m])])
+    return dict(loss=np.array([loss], np.float32), logits=dump_sample(eng.logits.cpu().numpy(), 1),
+                grads=dump_sample(flat(eng.export_grads()), 2), params=dump_sample(flat(eng.export_params()), 3))
 
 
 CPU_THREAD_CAP = 32      # the box reports 128 logical CPUs shared with other tenants; 128 torch threads thrash (6-52 tok/s)
@@ -238,6 +267,8 @@ def run_decode_bench(args, cfgd):
     wall_s = time.perf_counter() - t0
     clocks = sampler.stop() if sampler else None
     launches = L.load().progen_launch_count() - c0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(ids=np.asarray(ids, np.float64)))     # the last generation's token ids
     t = torch.tensor([dev_s, wall_s], device='cuda')
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -403,7 +434,13 @@ def main():
     ap.add_argument('--batch', type=int, default=None, help='per-GPU batch override')
     ap.add_argument('--fp32', action='store_true', help='fp32 engine (parity path) instead of bf16')
     ap.add_argument('--no-cpu-baseline', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed step computed to DIR/<name>.npy (float32 / float64, seeded samples of large arrays)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs writes the outputs of the b200 implementation')
     args.warmup = max(3, args.warmup) if args.impl == 'b200' else args.warmup
     cfgd = CONFIGS[args.config]
     kw = cfgd['kwargs']
@@ -498,6 +535,8 @@ def main():
     if world > 1:
         dist.all_reduce(loss_t)                        # per-rank losses are pre-scaled by 1/global_batch: the sum is the mean
     final_loss = float(loss_t.item())
+    if args.dump_outputs and rank == 0:                # before the legs below train further
+        dump_outputs(args.dump_outputs, train_step_outputs(eng, final_loss))
 
     # ---------------- end-to-end leg: public API with HOST (pinned) buffers, H2D + loss D2H inside the timed region.
     # Two readers of the per-step loss: (a) a training loop that keeps the GPU fed — `Trainer.step(host_batch)` returns the

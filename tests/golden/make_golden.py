@@ -1,8 +1,7 @@
-"""Generate tests/golden/*.npz by EXECUTING THE REFERENCE'S OWN SOURCE (/root/reference/progen_transformer/
-{progen,utils}.py, unmodified) under the numpy stand-ins in oracle/ref_shim/ (jax/haiku are not installable).
-
-Run in the dev container only (the GPU box has no /root/reference):
-    python tests/golden/make_golden.py
+"""Generate tests/golden/*.npz by EXECUTING THE REFERENCE'S OWN SOURCE (progen_transformer/{progen,utils}.py of a
+lucidrains/progen checkout, unmodified) under the numpy stand-ins in oracle/ref_shim/ (jax/haiku are not installable).
+The tests only read the stored files; regenerating needs the checkout:
+    python tests/golden/make_golden.py PATH_TO_LUCIDRAINS_PROGEN
 
 For each case the parameters come from the oracle's seeded initialiser (`init_params` + `randomize_params`,
 numpy default_rng => reproducible), are fed to the reference `model.apply`, and the reference's logits, loss
@@ -46,14 +45,14 @@ def make_inputs(kwargs, pseed, dseed, B=2):
     return cfg, params, data
 
 
-def main():
+def main(reference_dir):
     from oracle import progen_ref as O
     from oracle import progen_torch as T
     inputs = {name: make_inputs(*spec) for name, spec in CASES.items()}
 
     # ---- reference source under the shim
     sys.path.insert(0, os.path.join(ROOT, 'oracle', 'ref_shim'))
-    sys.path.insert(0, '/root/reference')
+    sys.path.insert(0, reference_dir)
     import haiku as hk
     from progen_transformer.progen import ProGen
     from progen_transformer import utils as RU
@@ -97,4 +96,6 @@ def main():
 
 
 if __name__ == '__main__':
-    main()
+    if len(sys.argv) != 2:
+        sys.exit('usage: python tests/golden/make_golden.py PATH_TO_LUCIDRAINS_PROGEN')
+    main(sys.argv[1])

@@ -1,4 +1,6 @@
-"""The drop-in CLIs end to end on a GPU: train.py (reference flags) on gzip TFRecords -> checkpoint -> resume -> sample.py."""
+"""The drop-in CLIs end to end on a GPU: train.py (reference flags) on gzip TFRecords -> checkpoint -> resume -> sample.py;
+bench.py's output dump."""
+import json
 import os
 import subprocess
 import sys
@@ -43,3 +45,29 @@ def test_train_checkpoint_resume_sample(tmp_path):
     out3 = run([os.path.join(ROOT, 'sample.py'), '--checkpoint_path', str(tmp_path / 'ckpts'), '--prime', '[tax=Mammalia] #',
                 '--greedy'], cwd=str(tmp_path))
     assert 'sequence length: 128' in out3 and '*' * 40 in out3
+
+
+def test_bench_dump_outputs_repeat(tmp_path):
+    """bench.py --dump-outputs: the last timed step's loss, logits, gradient and parameters as float .npy files of at most
+    64 MB, the same in two runs with the same arguments (seeded inputs; only the order of atomic reductions may differ)"""
+    import numpy as np
+    dumps = []
+    for r in range(2):
+        d = tmp_path / f'run{r}'
+        out = run([os.path.join(ROOT, 'bench.py'), '--config', 'tiny', '--steps', '2', '--warmup', '1', '--no-cpu-baseline',
+                   '--dump-outputs', str(d)], cwd=str(tmp_path))
+        lines = [l for l in out.splitlines() if l.strip()]
+        assert len(lines) == 1
+        j = json.loads(lines[0])
+        assert j['steps'] == 2
+        files = sorted(d.iterdir())
+        assert [f.name for f in files] == ['grads.npy', 'logits.npy', 'loss.npy', 'params.npy']
+        assert sum(f.stat().st_size for f in files) <= 64 << 20
+        arrays = {f.stem: np.load(f) for f in files}
+        assert all(a.dtype in (np.float32, np.float64) and a.size > 0 and np.isfinite(a).all() for a in arrays.values())
+        assert abs(float(arrays['loss'][0]) - j['final_loss']) <= 1e-6 * abs(j['final_loss'])
+        dumps.append(arrays)
+    a, b = dumps
+    for k in a:
+        assert a[k].shape == b[k].shape, k
+        assert np.abs(a[k] - b[k]).max() <= 1e-2 * max(1e-6, float(np.abs(a[k]).max())), k
