@@ -125,6 +125,13 @@ int progen_local_attn_fwd_tc(const void* qkv, void* out, float* lse, int B, int 
 int progen_local_attn_bwd_tc(const void* qkv, const void* out, const void* dout, const float* lse, void* dqkv, float* delta,
                              const float* rot_sin, const float* rot_cos, int B, int seq_len, int window, int heads, int dim_head,
                              void* stream);
+/* Same, with the rotary tables also given transposed (rot_sin_t / rot_cos_t: [dim_head/2, seq_len], or both null; the
+ * [seq_len, dim_head/2] tables are then required too) and the kernel variant chosen per call: mode 0 round-1 kernels,
+ * 1 / 2 / 3 round-2 kernels (3: gradient tiles stored through TMA, reading the transposed tables), -1 the
+ * PROGEN_ATTN_BWD_TS environment variable (default 3).  All modes compute the same gradients. */
+int progen_local_attn_bwd_tc_ex(const void* qkv, const void* out, const void* dout, const float* lse, void* dqkv, float* delta,
+                                const float* rot_sin, const float* rot_cos, const float* rot_sin_t, const float* rot_cos_t, int B,
+                                int seq_len, int window, int heads, int dim_head, int mode, void* stream);
 
 /* SGU gating — progen.py:182-184: out = xs * (Gp + spatial_biases[m]) and its backward (dxs, dGp, dbias) */
 int progen_sgu_gate_fwd(const void* xs, long long ldx, const void* gp, long long ldg, const float* bias, void* out,

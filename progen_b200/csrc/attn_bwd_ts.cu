@@ -22,6 +22,16 @@
 //   dQ  kernel (runs first; also writes delta = rowsum(dO o O) for the dK/dV kernel):
 //        S = Q K_j^T, dP = dO V_j^T (128 x 64 x 64)  ->  dS = exp2(S c - lse) o (dP - delta)  ->  dQ += dS K_j
 //   dKV kernel:  S^T = K Q_j^T, dP^T = V dO_j^T  ->  P^T, dS^T  ->  dV += P^T dO_j,  dK += dS^T Q_j
+//
+// Gradient stores (template flag TMA_ST, mode 3).  Without it every element-wise thread un-rotates and writes its own
+// row (store_grad_row): 128 B per thread with rows 3 KiB apart in dqkv, and the [n, 32] rotary tables read 64 B per thread
+// from 32 different lines per warp.  With it, each group stages its half of the finished tiles in shared memory (bf16,
+// 64-byte TMA swizzle: conflict-free 16-byte row writes) and one thread of the group writes them with a TMA store; the
+// rotary tables are read transposed ([32, n]: a warp's 32 consecutive positions are one 128-byte line per pair index).
+// Each group owns its own staging slot and issues its own boxes (128 rows x 32 channels): the two groups run a step
+// apart, and a shared 64-channel box would make the earlier group wait for the later one at every item.  In the dK/dV
+// kernel group g stores channels [32 g, 32 g + 32) of both dK and dV (one TMEM read-out of 2 x 32 columns per thread, as
+// with one whole 64-channel gradient per group).
 #include "tc_ptx.cuh"
 #include "../../include/progen_b200.h"
 
@@ -48,11 +58,13 @@ struct BwdDev {
   const float* lse;      // [T, h]
   float* delta;          // [T, h]   written by the dQ kernel, read by the dKV kernel
   bf16* dqkv;            // [T, 3I]
-  const float* rot_sin;  // [n, 32] or null
+  const float* rot_sin;  // entry (position p, pair j) at [p * rot_ld_pos + j * rot_ld_pair], or null
   const float* rot_cos;
+  int rot_ld_pos, rot_ld_pair;   // [n, 32]: 32, 1;  transposed [32, n]: 1, n
 };
 
 // store 32 fp32 gradient values of one row (channels ch0..ch0+31 of one head) as bf16, un-rotating pairs when tables given
+// (row-major [n, 32] tables: the launcher gives these kernels no other layout)
 __device__ __forceinline__ void store_grad_row(const BwdDev& a, bf16* dst, int pos, int ch0, const float (&v)[32]) {
   float o[32];
   if (a.rot_sin) {
@@ -73,6 +85,44 @@ __device__ __forceinline__ void store_grad_row(const BwdDev& a, bf16* dst, int p
   store_vec<32>(dst, o);
 }
 
+// ---------------------------------------------------------------------------------------- TMA-store epilogue (TMA_ST)
+constexpr int ST_BOX_BYTES = RB * 32 * 2;      // 8 KiB: 128 rows x 32 bf16 channels, 64-byte rows
+
+// un-rotate 32 fp32 values of one row (channels ch0..ch0+31 of one head, position pos) in place when tables are given
+__device__ __forceinline__ void unrotate32(const BwdDev& a, int pos, int ch0, float (&v)[32]) {
+  if (!a.rot_sin) return;
+  const long long e0 = (long long)pos * a.rot_ld_pos + (long long)(ch0 >> 1) * a.rot_ld_pair;
+  float s[16], c[16];
+#pragma unroll
+  for (int i = 0; i < 16; ++i) {
+    s[i] = __ldg(a.rot_sin + e0 + (long long)i * a.rot_ld_pair);
+    c[i] = __ldg(a.rot_cos + e0 + (long long)i * a.rot_ld_pair);
+  }
+#pragma unroll
+  for (int i = 0; i < 16; ++i) {                         // d/d(x0,x1) of (x0 c - x1 s, x1 c + x0 s)
+    const float x0 = v[2 * i], x1 = v[2 * i + 1];
+    v[2 * i] = x0 * c[i] + x1 * s[i];
+    v[2 * i + 1] = x1 * c[i] - x0 * s[i];
+  }
+}
+
+// row `row` of a [128 x 32] bf16 staging box in the 64-byte TMA swizzle (16-byte chunk c of row r at chunk
+// c ^ ((r >> 1) & 3); the box is 1024-byte aligned): 8 consecutive rows cover all 32 banks
+__device__ __forceinline__ void stage_row32(uint32_t box, int row, const float (&v)[32]) {
+#pragma unroll
+  for (int c = 0; c < 4; ++c)
+    asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};"
+                 ::"r"(box + row * 64 + ((c ^ ((row >> 1) & 3)) << 4)), "r"(pack_bf16x2(v[8 * c], v[8 * c + 1])),
+                   "r"(pack_bf16x2(v[8 * c + 2], v[8 * c + 3])), "r"(pack_bf16x2(v[8 * c + 4], v[8 * c + 5])),
+                   "r"(pack_bf16x2(v[8 * c + 6], v[8 * c + 7])) : "memory");
+}
+
+// the 128 threads of element-wise group g (warps 4 + 4 g .. 7 + 4 g)
+__device__ __forceinline__ void group_bar(int g) {
+  if (g == 0) asm volatile("bar.sync 1, 128;" ::: "memory");
+  else asm volatile("bar.sync 2, 128;" ::: "memory");
+}
+
 // ===================================================================================================== dK, dV
 namespace dkv {
 constexpr int OFF_KV = 0;                                                      // [kvb]: K tile, V tile (128 rows each)
@@ -81,6 +131,9 @@ constexpr int OFF_STAT = OFF_QS + NS * STAGE_BYTES;                            /
 constexpr int STAT_BYTES = 2 * CT * 4;
 constexpr int OFF_BAR = OFF_STAT + NS * STAT_BYTES;
 constexpr int SMEM_BYTES = OFF_BAR + 256 + 1024;
+constexpr int OFF_ST = (OFF_BAR + 256 + 1023) / 1024 * 1024;                   // TMA_ST: [group]: dK box, dV box
+constexpr int SMEM_BYTES_ST = OFF_ST + 2 * 2 * ST_BOX_BYTES + 1024;            // 196 KiB with NS = 6
+static_assert(SMEM_BYTES_ST <= 227 * 1024, "dK/dV staging slots do not fit");
 }  // namespace dkv
 
 // one work item = (batch, head, 128-key tile); its steps are the 64-query tiles that can see those keys: own window
@@ -101,9 +154,11 @@ __device__ __forceinline__ bool decode_kitem(const BwdDev& a, int wi, KItem& it)
   return true;
 }
 
+template <bool TMA_ST>
 __global__ void __launch_bounds__(384, 1) attn_bwd_dkv_ts_kernel(const __grid_constant__ CUtensorMap tmap_qkv_row,
                                                                 const __grid_constant__ CUtensorMap tmap_qkv_col,
-                                                                const __grid_constant__ CUtensorMap tmap_do_col, const BwdDev a) {
+                                                                const __grid_constant__ CUtensorMap tmap_do_col,
+                                                                const __grid_constant__ CUtensorMap tmap_dqkv_st, const BwdDev a) {
   using namespace dkv;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -121,7 +176,10 @@ __global__ void __launch_bounds__(384, 1) attn_bwd_dkv_ts_kernel(const __grid_co
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int I = a.h * DH;
 
-  if (warp == 0 && lane == 0) { prefetch_tensormap(&tmap_qkv_row); prefetch_tensormap(&tmap_qkv_col); prefetch_tensormap(&tmap_do_col); }
+  if (warp == 0 && lane == 0) {
+    prefetch_tensormap(&tmap_qkv_row); prefetch_tensormap(&tmap_qkv_col); prefetch_tensormap(&tmap_do_col);
+    if (TMA_ST) prefetch_tensormap(&tmap_dqkv_st);
+  }
   if (warp == 1 && lane == 0) {
     for (int b = 0; b < 2; ++b) { mbar_init(kv_full(b), 1); mbar_init(kv_empty(b), 1); }
     for (int s = 0; s < NS; ++s) { mbar_init(qs_full(s), 2); mbar_init(qs_empty(s), 1); }   // full: TMA bytes + the stats warp
@@ -268,6 +326,38 @@ __global__ void __launch_bounds__(384, 1) attn_bwd_dkv_ts_kernel(const __grid_co
     int pend_b = 0, pend_hh = 0, pend_k0 = 0;
     uint32_t pend_item = 0;
     auto epilogue = [&]() {     // group 0 stores dK (x 1/sqrt(dh)), group 1 stores dV
+      if constexpr (TMA_ST) {   // group g: channels [32 g, 32 g + 32) of dK (x 1/sqrt(dh)) and of dV, both un-rotated
+        const uint32_t slot = base + OFF_ST + g * (2 * ST_BOX_BYTES);
+        mbar_wait(acc_full, pend_item & 1);
+        tcgen05_fence_after();
+        uint32_t rk[32], rv[32];
+        tmem_ld32_issue(tmem_base + lane_addr + 384 + 32 * g, rk);
+        tmem_ld32_issue(tmem_base + lane_addr + 448 + 32 * g, rv);
+        tmem_ld32_wait(rk);
+        tmem_ld32_wait(rv);
+        tcgen05_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(acc_empty);
+        float vk[32], vv[32];
+#pragma unroll
+        for (int i = 0; i < 32; ++i) { vk[i] = __uint_as_float(rk[i]) * SCALE; vv[i] = __uint_as_float(rv[i]); }
+        unrotate32(a, pend_k0 + row, 32 * g, vk);
+        unrotate32(a, pend_k0 + row, 32 * g, vv);                            // v is rotated too (progen.py:36-41)
+        if (row == 0) bulk_wait_group_read<0>();                             // the previous item's boxes have left the slot
+        group_bar(g);
+        stage_row32(slot, row, vk);
+        stage_row32(slot + ST_BOX_BYTES, row, vv);
+        fence_proxy_async();                                                 // my slot writes -> visible to the TMA store
+        group_bar(g);
+        if (row == 0) {
+          const int r0 = pend_b * a.n + pend_k0, c0 = pend_hh * DH + 32 * g;
+          tma_store_2d(&tmap_dqkv_st, slot, I + c0, r0);
+          tma_store_2d(&tmap_dqkv_st, slot + ST_BOX_BYTES, 2 * I + c0, r0);
+          bulk_commit_group();
+        }
+        pending = false;
+        return;
+      }
       mbar_wait(acc_full, pend_item & 1);
       tcgen05_fence_after();
       const long long tr = (long long)pend_b * a.n + pend_k0 + row;
@@ -340,6 +430,7 @@ __global__ void __launch_bounds__(384, 1) attn_bwd_dkv_ts_kernel(const __grid_co
       pend_b = it.b; pend_hh = it.hh; pend_k0 = it.k0; pend_item = item; pending = true;
     }
     if (pending) epilogue();
+    if (TMA_ST && row == 0) bulk_wait_group<0>();                            // every store has completed before smem goes away
   }
   tcgen05_fence_before();
   __syncthreads();
@@ -353,6 +444,9 @@ constexpr int OFF_KV = 4 * ROW_TILE_BYTES;                                     /
 constexpr int OFF_BAR = OFF_KV + NS * STAGE_BYTES;
 constexpr int OFF_RC = OFF_BAR + 256;                                          // [qb][-delta | -lse*log2e][128] row constants
 constexpr int SMEM_BYTES = OFF_RC + 2 * 2 * RB * 4 + 1024;
+constexpr int OFF_ST = (OFF_RC + 2 * 2 * RB * 4 + 1023) / 1024 * 1024;        // TMA_ST: [group]: dQ box
+constexpr int SMEM_BYTES_ST = OFF_ST + 2 * ST_BOX_BYTES + 1024;
+static_assert(SMEM_BYTES_ST <= 227 * 1024, "dQ staging slots do not fit");
 }  // namespace dq
 
 // one work item = (batch, head, 128-query tile); steps = the visible 64-key tiles (look-back window, then own window up to
@@ -372,10 +466,11 @@ __device__ __forceinline__ bool decode_qitem(const BwdDev& a, int wi, QItem& it)
   return true;
 }
 
-template <bool POLY>
+template <bool POLY, bool TMA_ST>
 __global__ void __launch_bounds__(384, 1) attn_bwd_dq_ts_kernel(const __grid_constant__ CUtensorMap tmap_qkv_row,
                                                                const __grid_constant__ CUtensorMap tmap_qkv_col,
-                                                               const __grid_constant__ CUtensorMap tmap_do_row, const BwdDev a) {
+                                                               const __grid_constant__ CUtensorMap tmap_do_row,
+                                                               const __grid_constant__ CUtensorMap tmap_dqkv_st, const BwdDev a) {
   using namespace dq;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -395,7 +490,10 @@ __global__ void __launch_bounds__(384, 1) attn_bwd_dq_ts_kernel(const __grid_con
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int I = a.h * DH;
 
-  if (warp == 0 && lane == 0) { prefetch_tensormap(&tmap_qkv_row); prefetch_tensormap(&tmap_qkv_col); prefetch_tensormap(&tmap_do_row); }
+  if (warp == 0 && lane == 0) {
+    prefetch_tensormap(&tmap_qkv_row); prefetch_tensormap(&tmap_qkv_col); prefetch_tensormap(&tmap_do_row);
+    if (TMA_ST) prefetch_tensormap(&tmap_dqkv_st);
+  }
   if (warp == 1 && lane == 0) {
     for (int b = 0; b < 2; ++b) { mbar_init(qd_full(b), 1); mbar_init(qd_empty(b), 1); }
     for (int s = 0; s < NS; ++s) { mbar_init(kv_full(s), 1); mbar_init(kv_empty(s), 1); }
@@ -564,8 +662,22 @@ __global__ void __launch_bounds__(384, 1) attn_bwd_dq_ts_kernel(const __grid_con
       float v0[32];
 #pragma unroll
       for (int i = 0; i < 32; ++i) v0[i] = __uint_as_float(r0[i]) * SCALE;
-      const long long t = (long long)pend_b * a.n + pend_q0 + row;
-      store_grad_row(a, a.dqkv + t * (3LL * I) + pend_hh * DH + g * 32, pend_q0 + row, g * 32, v0);
+      if constexpr (TMA_ST) {
+        const uint32_t slot = base + OFF_ST + g * ST_BOX_BYTES;
+        unrotate32(a, pend_q0 + row, g * 32, v0);
+        if (row == 0) bulk_wait_group_read<0>();                             // the previous item's box has left the slot
+        group_bar(g);
+        stage_row32(slot, row, v0);
+        fence_proxy_async();
+        group_bar(g);
+        if (row == 0) {
+          tma_store_2d(&tmap_dqkv_st, slot, pend_hh * DH + g * 32, pend_b * a.n + pend_q0);
+          bulk_commit_group();
+        }
+      } else {
+        const long long t = (long long)pend_b * a.n + pend_q0 + row;
+        store_grad_row(a, a.dqkv + t * (3LL * I) + pend_hh * DH + g * 32, pend_q0 + row, g * 32, v0);
+      }
       pending = false;
     };
     for (int wi = blockIdx.x; decode_qitem(a, wi, it); wi += gridDim.x, ++item) {
@@ -618,6 +730,7 @@ __global__ void __launch_bounds__(384, 1) attn_bwd_dq_ts_kernel(const __grid_con
       pend_b = it.b; pend_hh = it.hh; pend_q0 = it.q0; pend_item = item; pending = true;
     }
     if (pending) epilogue();
+    if (TMA_ST && row == 0) bulk_wait_group<0>();
   }
   tcgen05_fence_before();
   __syncthreads();
@@ -627,10 +740,18 @@ __global__ void __launch_bounds__(384, 1) attn_bwd_dq_ts_kernel(const __grid_con
 }  // namespace
 
 // Round-2 backward (both kernels); returns 1 when disabled so the caller falls back to the round-1 kernels.
+// mode: 0 off, 1 MUFU only, 2 + FMA-pipe exp2 in dQ, 3 = 2 + gradient tiles stored through TMA (see the file header);
+// -1 reads PROGEN_ATTN_BWD_TS (once per process; default 3).  Rotary tables: row-major [n, 32] (rot_sin / rot_cos) and/or
+// transposed [32, n] (rot_sin_t / rot_cos_t); modes 1 and 2 read the row-major ones, mode 3 the transposed ones when given.
 int attn_bwd_ts_launch(const void* qkv, const void* out, const void* dout, const float* lse, void* dqkv, float* delta,
-                       const float* rot_sin, const float* rot_cos, int B, int seq_len, int window, int heads, cudaStream_t s) {
-  static int mode = [] { const char* e = getenv("PROGEN_ATTN_BWD_TS"); return e ? atoi(e) : 2; }();   // 0 off, 1 MUFU only, 2 + FMA-pipe exp2 in dQ
+                       const float* rot_sin, const float* rot_cos, const float* rot_sin_t, const float* rot_cos_t, int B,
+                       int seq_len, int window, int heads, int mode, cudaStream_t s) {
+  static const int env_mode = [] { const char* e = getenv("PROGEN_ATTN_BWD_TS"); return e ? atoi(e) : 3; }();
+  if (mode < 0) mode = env_mode;
   if (!mode || window % RB != 0) return 1;
+  PG_CHECK_ARG(mode <= 3);
+  const bool tma_st = mode == 3;
+  PG_CHECK_ARG(tma_st || rot_sin || !rot_sin_t);      // modes 1 and 2 have no transposed-table path
   const long long T = (long long)B * seq_len;
   const int I = heads * DH;
   CUtensorMap tq_row, tq_col, tdo_row, tdo_col;
@@ -642,20 +763,32 @@ int attn_bwd_ts_launch(const void* qkv, const void* out, const void* dout, const
   if (rc) return rc;
   rc = pg_tensor_map_2d_bf16(dout, (uint64_t)I, (uint64_t)T, (uint64_t)I, DH, CT, &tdo_col);
   if (rc) return rc;
+  CUtensorMap tst;                                      // dqkv, 128 rows x 32 channels per box, 64-byte swizzle
+  if (tma_st) {
+    rc = pg_tensor_map_2d(dqkv, 2, 3ull * I, (uint64_t)T, 3ull * I, 32, RB, 64, &tst);
+    if (rc) return rc;
+  } else {
+    tst = tq_row;                                       // not read
+  }
   static bool once = false;
   if (!once) {
-    PG_CUDA(cudaFuncSetAttribute(attn_bwd_dq_ts_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, dq::SMEM_BYTES));
-    PG_CUDA(cudaFuncSetAttribute(attn_bwd_dq_ts_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dq::SMEM_BYTES));
-    PG_CUDA(cudaFuncSetAttribute(attn_bwd_dkv_ts_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, dkv::SMEM_BYTES));
+    PG_CUDA(cudaFuncSetAttribute(attn_bwd_dq_ts_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, dq::SMEM_BYTES));
+    PG_CUDA(cudaFuncSetAttribute(attn_bwd_dq_ts_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, dq::SMEM_BYTES));
+    PG_CUDA(cudaFuncSetAttribute(attn_bwd_dq_ts_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dq::SMEM_BYTES_ST));
+    PG_CUDA(cudaFuncSetAttribute(attn_bwd_dkv_ts_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, dkv::SMEM_BYTES));
+    PG_CUDA(cudaFuncSetAttribute(attn_bwd_dkv_ts_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dkv::SMEM_BYTES_ST));
     once = true;
   }
-  BwdDev a{B, seq_len, window, heads, (const bf16*)out, (const bf16*)dout, lse, delta, (bf16*)dqkv, rot_sin, rot_cos};
+  BwdDev a{B, seq_len, window, heads, (const bf16*)out, (const bf16*)dout, lse, delta, (bf16*)dqkv, rot_sin, rot_cos, DH / 2, 1};
+  if (tma_st && rot_sin_t) { a.rot_sin = rot_sin_t; a.rot_cos = rot_cos_t; a.rot_ld_pos = 1; a.rot_ld_pair = seq_len; }
   const long long items = (long long)B * heads * (seq_len / RB);
   const int grid = (int)(items < pg_num_sms() ? items : pg_num_sms());
-  if (mode >= 2) attn_bwd_dq_ts_kernel<true><<<grid, 384, dq::SMEM_BYTES, s>>>(tq_row, tq_col, tdo_row, a);
-  else attn_bwd_dq_ts_kernel<false><<<grid, 384, dq::SMEM_BYTES, s>>>(tq_row, tq_col, tdo_row, a);
+  if (tma_st) attn_bwd_dq_ts_kernel<true, true><<<grid, 384, dq::SMEM_BYTES_ST, s>>>(tq_row, tq_col, tdo_row, tst, a);
+  else if (mode == 2) attn_bwd_dq_ts_kernel<true, false><<<grid, 384, dq::SMEM_BYTES, s>>>(tq_row, tq_col, tdo_row, tst, a);
+  else attn_bwd_dq_ts_kernel<false, false><<<grid, 384, dq::SMEM_BYTES, s>>>(tq_row, tq_col, tdo_row, tst, a);
   PG_LAUNCH_CHECK();
-  attn_bwd_dkv_ts_kernel<<<grid, 384, dkv::SMEM_BYTES, s>>>(tq_row, tq_col, tdo_col, a);
+  if (tma_st) attn_bwd_dkv_ts_kernel<true><<<grid, 384, dkv::SMEM_BYTES_ST, s>>>(tq_row, tq_col, tdo_col, tst, a);
+  else attn_bwd_dkv_ts_kernel<false><<<grid, 384, dkv::SMEM_BYTES, s>>>(tq_row, tq_col, tdo_col, tst, a);
   PG_LAUNCH_CHECK();
   return PROGEN_OK;
 }

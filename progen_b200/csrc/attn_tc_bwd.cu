@@ -15,7 +15,8 @@
 #include "../../include/progen_b200.h"
 
 int attn_bwd_ts_launch(const void* qkv, const void* out, const void* dout, const float* lse, void* dqkv, float* delta,
-                       const float* rot_sin, const float* rot_cos, int B, int seq_len, int window, int heads, cudaStream_t s);
+                       const float* rot_sin, const float* rot_cos, const float* rot_sin_t, const float* rot_cos_t, int B,
+                       int seq_len, int window, int heads, int mode, cudaStream_t s);
 
 namespace {
 
@@ -490,12 +491,14 @@ __global__ void __launch_bounds__(384, 1) attn_bwd_dkv_tc_kernel(const __grid_co
 extern "C" {
 
 // tcgen05 backward; same contract as progen_local_attn_bwd (delta is produced by the dQ kernel), window % 128 == 0.
-int progen_local_attn_bwd_tc(const void* qkv, const void* out, const void* dout, const float* lse, void* dqkv, float* delta,
-                             const float* rot_sin, const float* rot_cos, int B, int seq_len, int window, int heads, int dim_head,
-                             void* stream) {
+int progen_local_attn_bwd_tc_ex(const void* qkv, const void* out, const void* dout, const float* lse, void* dqkv, float* delta,
+                                const float* rot_sin, const float* rot_cos, const float* rot_sin_t, const float* rot_cos_t, int B,
+                                int seq_len, int window, int heads, int dim_head, int mode, void* stream) {
   PG_CHECK_ARG(B > 0 && heads > 0 && dim_head == DH && window % 128 == 0 && seq_len % window == 0);
+  PG_CHECK_ARG(!rot_sin == !rot_cos && !rot_sin_t == !rot_cos_t && (rot_sin || !rot_sin_t));
   // round-2 kernels (element-wise results in tensor memory, alternating groups; attn_bwd_ts.cu)
-  const int rc_ts = attn_bwd_ts_launch(qkv, out, dout, lse, dqkv, delta, rot_sin, rot_cos, B, seq_len, window, heads, (cudaStream_t)stream);
+  const int rc_ts = attn_bwd_ts_launch(qkv, out, dout, lse, dqkv, delta, rot_sin, rot_cos, rot_sin_t, rot_cos_t, B, seq_len,
+                                       window, heads, mode, (cudaStream_t)stream);
   if (rc_ts <= 0) return rc_ts;
   const long long T = (long long)B * seq_len;
   const int I = heads * DH;
@@ -541,6 +544,13 @@ int progen_local_attn_bwd_tc(const void* qkv, const void* out, const void* dout,
   attn_bwd_dkv_tc_kernel<<<grid, 384, dkv::SMEM_BYTES, s>>>(tq_row, tq_col, tdo_col, a);
   PG_LAUNCH_CHECK();
   return PROGEN_OK;
+}
+
+int progen_local_attn_bwd_tc(const void* qkv, const void* out, const void* dout, const float* lse, void* dqkv, float* delta,
+                             const float* rot_sin, const float* rot_cos, int B, int seq_len, int window, int heads, int dim_head,
+                             void* stream) {
+  return progen_local_attn_bwd_tc_ex(qkv, out, dout, lse, dqkv, delta, rot_sin, rot_cos, nullptr, nullptr, B, seq_len, window,
+                                     heads, dim_head, -1, stream);
 }
 
 }  // extern "C"

@@ -141,6 +141,9 @@ class Engine:
         ang = np.arange(n, dtype=np.float64)[:, None] * inv_freq[None, :]
         self.rot_sin = torch.tensor(np.sin(ang), **f32).contiguous()
         self.rot_cos = torch.tensor(np.cos(ang), **f32).contiguous()
+        # the same, [dim_head/2, n]: the attention backward reads them one position per thread (coalesced)
+        self.rot_sin_t = self.rot_sin.t().contiguous()
+        self.rot_cos_t = self.rot_cos.t().contiguous()
         self.B = 0
         self.loss = torch.zeros(1, device=self.dev)       # exists before the first batch: a rank without rows still reports 0
         self.loaded_token = None
@@ -363,8 +366,14 @@ class Engine:
 
     def attn_bwd(self, qkv, out, dout, lse, dqkv):
         if self.attn_tc:
-            fn = self.lib.progen_local_attn_bwd_tc if self.attn_bwd_kind == 'tcgen05' else self.lib.progen_local_attn_bwd
-            L.check(fn(qkv.data_ptr(), out.data_ptr(), dout.data_ptr(), lse.data_ptr(), dqkv.data_ptr(),
+            if self.attn_bwd_kind == 'tcgen05':
+                L.check(self.lib.progen_local_attn_bwd_tc_ex(qkv.data_ptr(), out.data_ptr(), dout.data_ptr(), lse.data_ptr(),
+                                                             dqkv.data_ptr(), self.delta.data_ptr(), self.rot_sin.data_ptr(),
+                                                             self.rot_cos.data_ptr(), self.rot_sin_t.data_ptr(),
+                                                             self.rot_cos_t.data_ptr(), self.B, self.n, self.w, self.h, self.dh, -1,
+                                                             L.stream()), 'local_attn_bwd')
+                return     # rotary backward is fused into the kernels' epilogues
+            L.check(self.lib.progen_local_attn_bwd(qkv.data_ptr(), out.data_ptr(), dout.data_ptr(), lse.data_ptr(), dqkv.data_ptr(),
                                                    self.delta.data_ptr(), self.rot_sin.data_ptr(), self.rot_cos.data_ptr(), self.B,
                                                    self.n, self.w, self.h, self.dh, L.stream()), 'local_attn_bwd')
             return     # rotary backward is fused into the kernel's epilogue

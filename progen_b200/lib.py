@@ -59,6 +59,7 @@ PROTOTYPES = {
     'progen_local_attn_fwd_tc': [_P, _P, _P, _I, _I, _I, _I, _I, _P],
     'progen_local_attn_bwd': [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P],
     'progen_local_attn_bwd_tc': [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P],
+    'progen_local_attn_bwd_tc_ex': [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P],
     'progen_sgu_gate_fwd': [_P, _LL, _P, _LL, _P, _P, _LL, _I, _LL, _I, _I, _P],
     'progen_sgu_gate_bwd': [_P, _LL, _P, _LL, _P, _LL, _P, _P, _LL, _P, _LL, _P, _I, _LL, _I, _I, _P],
     'progen_gelu_bwd': [_P, _P, _I, _LL, _P],
